@@ -43,11 +43,35 @@ def parse():
     ap.add_argument("--nprot", type=int, default=680000, help="synthetic DB size (680000 = viruses scale)")
     ap.add_argument("--reads", type=int, default=10_000_000, help="read pairs per GPU per step")
     ap.add_argument("--cpu-sample", type=int, default=0, help="pairs for the CPU baseline sample (0 = auto)")
-    ap.add_argument("--workdir", default=os.environ.get("KJ_BENCH_DIR", "/tmp/kjbench"))
+    ap.add_argument("--workdir", default=os.environ.get("KJ_BENCH_DIR", os.path.join(tempfile.gettempdir(), "kjbench")))
     ap.add_argument("--skip-cpu", action="store_true", help="no CPU legs (roofline numerator, cpu_baseline, parity)")
     ap.add_argument("--headline-only", action="store_true", help="skip the `configs` sub-runs (greedy, large_index)")
     ap.add_argument("--large-rows", type=float, default=2.7e10, help="target BWT rows of the large_index config (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline device-resident path returned in its last timed step to DIR/<name>.npy (float64, a seeded "
+                         "sample of this rank's reads; with several GPUs also a sample of the all-gathered dense taxon indices of every rank)")
     return ap.parse_args()
+
+
+DUMP_SAMPLE = 1 << 20          # reads in a --dump-outputs sample: at most 6 arrays x 8 bytes x 2^20 = 48 MB
+
+
+def dump_outputs(R, directory):
+    """Per-read results of the last timed device-resident step of the headline configuration (kj_classify_device2): taxon id, best
+    match length/score and dense taxon index, for a fixed seeded sample of the reads (all of them if the batch is small enough), with
+    the sampled read indices.  With several GPUs, also a seeded sample of the all-gathered dense indices of every rank's reads (the
+    job's whole output).  float64 holds every value exactly (ids and indices < 2^53)."""
+    os.makedirs(directory, exist_ok=True)
+    def sample(n):
+        return np.arange(n, dtype=np.int64) if n <= DUMP_SAMPLE else np.sort(np.random.default_rng(12345).choice(n, DUMP_SAMPLE, replace=False))
+    idx = sample(R.n)
+    out = {"read_index": idx, "taxon": R.kept["taxon"].cpu().numpy().view(np.uint64)[idx], "best": R.kept["best"].cpu().numpy().view(np.uint32)[idx],
+           "dense_taxon_index": R.kept["dense_taxon_index"].cpu().numpy().view(np.uint32)[idx]}
+    if R.kept["gathered"] is not None:
+        g = R.kept["gathered"].cpu().numpy().view(np.uint32); gidx = sample(len(g))
+        out.update({"all_ranks_read_index": gidx, "all_ranks_dense_taxon_index": g[gidx]})
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a.astype(np.float64))
 
 
 def build_workload(args, rank):
@@ -231,7 +255,7 @@ class Runner:
         self.gather_done[k] = done
 
     def step_device(self, clf):
-        k = self.i & 1; self.i += 1
+        k = self.i & 1; self.i += 1; self.last_k = k
         if self.dist and self.gather_done[k] is not None:
             self.stream.wait_event(self.gather_done[k])                # buffer k is free again once its previous gather has finished
         d = self.d
@@ -277,11 +301,17 @@ class Runner:
         return float(t.item()), clf.kernel_launches - l0
 
 
-def measure(R, clf, steps, warmup, world):
-    """value (device-resident) and e2e (host buffers) of one configuration on runner R."""
+def measure(R, clf, steps, warmup, world, keep=False):
+    """value (device-resident) and e2e (host buffers) of one configuration on runner R, `steps` timed steps each.  keep: R.kept = the
+    device outputs of the last device-resident step (untimed copies, taken before the e2e leg reuses the buffers)."""
     ms_dev, launches = R.timed(clf, R.step_device, steps, max(3, warmup))
+    if keep:
+        k = R.last_k
+        R.kept = {"taxon": R.d_tax.clone(), "best": R.d_best.clone(), "dense_taxon_index": R.d_compact[k].clone(),
+                  "gathered": R.gathered[k].clone() if R.dist else None}
+        R.torch.cuda.synchronize()
     kernel_ms = clf.last_kernel_ms                                   # CUDA events around the last classify kernel, on its launch stream
-    e2e_steps = max(2, steps // 2)
+    e2e_steps = steps
     ms_host, _ = R.timed(clf, R.step_host, e2e_steps, 1)
     clf.check_errors()
     assert R.torch.equal(R.h_tax, R.d_tax.cpu()), "host-buffer and device-buffer entry points disagree"
@@ -366,8 +396,10 @@ def main():
     R = Runner(torch, dist, world, local, *db.reads(7, rank * n, n, 150, True))      # this rank's shard of the job: items [rank*n, (rank+1)*n)
 
     sampler = ClockSampler(local); sampler.start()
-    res = measure(R, clf, args.steps, args.warmup, world)
+    res = measure(R, clf, args.steps, args.warmup, world, keep=bool(args.dump_outputs))
     sampler.stop_flag = True; sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(R, args.dump_outputs)
     # untimed: the kaiju2table-style summary -- per-taxon read counts in HBM, one all-reduce across the ranks (SURVEY.md 8e); and the
     # dense indices the ranks gathered map back to the 64-bit ids
     clf.counts_reset(); clf.counts_add_device(R.d_tax.data_ptr(), n); torch.cuda.synchronize()
@@ -387,8 +419,8 @@ def main():
     if dist:   # strong scaling: the 10 M-pair job of ONE GPU split over the ranks (reads [0, n) of the same stream)
         lo, hi = rank * n // world, (rank + 1) * n // world
         RS = Runner(torch, dist, world, local, *db.reads(7, lo, hi - lo, 150, True))
-        ms_s, _ = RS.timed(clf, RS.step_device, max(2, args.steps // 2), 2)
-        strong = {"value": n * max(2, args.steps // 2) / (ms_s / 1000.0), "unit": "read pairs/s", "total_pairs": n, "note": "fixed job of %d pairs split over %d GPUs, device-resident, gather included" % (n, world)}
+        ms_s, _ = RS.timed(clf, RS.step_device, args.steps, 2)
+        strong = {"value": n * args.steps / (ms_s / 1000.0), "unit": "read pairs/s", "total_pairs": n, "note": "fixed job of %d pairs split over %d GPUs, device-resident, gather included" % (n, world)}
         del RS
 
     line = None
@@ -417,7 +449,7 @@ def main():
         mem_tax = R.h_tax.numpy().view(np.uint64).copy() if args.mode == "mem" else None
         try:
             clf.set_params(kb.make_params(other, m=11))
-            sub = measure(R, clf, max(2, args.steps // 2), 3, 1)
+            sub = measure(R, clf, args.steps, 3, 1)
             sub.update({"workload": "configs[2]: %s -e 3 -s 65 -m 11 (E-value 0.01, SEG on), the same %d PE150 pairs vs synth-viruses .fmi" % (other.upper(), n) if other == "greedy" else "MEM -m 11"})
             if not args.skip_cpu:
                 cpu_legs(R, sub, other, db, fmi, nodes, args)
@@ -451,7 +483,7 @@ def large_index(kb, torch, R, clf_base, fmi, nodes, mem_tax, args, local, alg_ba
     big = kb.Classifier(fmi, nodes, device=local, params=kb.make_params("mem", m=11), copies=copies)
     t_create = time.time() - t0
     try:
-        sub = measure(R, big, 2, 3, 1)
+        sub = measure(R, big, args.steps, 3, 1)
         tax = R.h_tax.numpy().view(np.uint64)
         diffs = int((tax != mem_tax).sum()) if mem_tax is not None else None
         peak, peak_src = peak_hbm()

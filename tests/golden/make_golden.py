@@ -40,10 +40,11 @@ def revcomp(s):
     return s[::-1].translate(str.maketrans("ACGTacgtN", "TGCAtgcaN"))
 
 
-def main():
+def write_db_faa(faa, nodes):
+    """The golden DB as FASTA + nodes.dmp (the input of db.fmi); returns the DB, the random generator in its state after the DB and
+    the adversarial proteins (capped, same, plain, zero, lowc)."""
     rnd = random.Random(20240607)
     db = SynthDB(800, 3)
-    faa, nodes = os.path.join(HERE, "db.faa"), os.path.join(HERE, "nodes.dmp")
     db.write(faa, nodes)
     node_ids = [int(l.split()[0]) for l in open(nodes)]
     leaves = [node_ids[5 + (i % (len(node_ids) - 5))] for i in range(200)]     # any node may carry proteins
@@ -66,6 +67,13 @@ def main():
         f.write(">MISSING_7777777\n%s\n" % zero[::-1])
         for i in range(3):
             f.write(">LOWC%d_%d\n%s\n" % (i, leaves[50 + i], lowc))
+    return db, rnd, (capped, same, plain, zero, lowc)
+
+
+def main():
+    faa, nodes = os.path.join(HERE, "db.faa"), os.path.join(HERE, "nodes.dmp")
+    db, rnd, (capped, same, plain, zero, lowc) = write_db_faa(faa, nodes)
+    aa = "ACDEFGHIKLMNPQRSTVWY"
     fmi = build_fmi(faa, os.path.join(HERE, "db"), threads=4)
     os.remove(faa)
 

@@ -238,10 +238,11 @@ def read_fastq_packed(path):
     return names, data, off
 
 
-def make_quirk_db(d, nprot=512, plen=255, seed=9, nreads=3000):
+def make_quirk_db(d, nprot=512, plen=255, seed=9, nreads=3000, build=False):
     """A DB whose BWT length is an exact multiple of 2^16 (nprot * (plen + 1) = 131072 rows by default): the case in which the
     reference's FM-index checkpoints misbehave for the last 129 positions (fmicommon.h:60-73, 88-89).  Returns (fmi, nodes, read
-    strings).  Needs oracle/_ref (index builder)."""
+    strings).  The index of the default DB is committed (tests/golden/quirk_db.fmi, built by the reference's kaiju-mkbwt/-mkfmi);
+    build=True builds it with oracle/_ref."""
     import random
     rnd = random.Random(seed); aa = "ACDEFGHIKLMNPQRSTVWY"
     assert (nprot * (plen + 1)) % 65536 == 0
@@ -253,7 +254,11 @@ def make_quirk_db(d, nprot=512, plen=255, seed=9, nreads=3000):
         f.write("1\t|\t1\t|\tno rank\t|\n")
         for t in range(100, 107):
             f.write("%d\t|\t1\t|\tspecies\t|\n" % t)
-    fmi = build_fmi(d + "/db.faa", d + "/db", threads=2)
+    if build:
+        fmi = build_fmi(d + "/db.faa", d + "/db", threads=2)
+    else:
+        assert (nprot, plen, seed) == (512, 255, 9), "only the default quirk DB has a committed index"
+        fmi = os.path.join(GOLDEN_DIR, "quirk_db.fmi")
     codon = {'A': 'GCT', 'R': 'CGT', 'N': 'AAT', 'D': 'GAT', 'C': 'TGT', 'Q': 'CAA', 'E': 'GAA', 'G': 'GGT', 'H': 'CAT', 'I': 'ATT',
              'L': 'CTG', 'K': 'AAA', 'M': 'ATG', 'F': 'TTT', 'P': 'CCT', 'S': 'TCT', 'T': 'ACT', 'W': 'TGG', 'Y': 'TAT', 'V': 'GTT'}
     reads = []

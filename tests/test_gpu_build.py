@@ -1,9 +1,12 @@
 """GPU tests of the index construction on the device (kj_build.h): array for array against the host transcoder, the scaled (K-fold) index
-against the index the reference's own kaiju-mkbwt/-mkfmi build for the K-fold FASTA, the dense-index output, and a genuinely wide index."""
-import os, tempfile
+against the index the reference's own kaiju-mkbwt/-mkfmi build for the K-fold FASTA (stored answers), the dense-index output, and a
+genuinely wide index."""
+import os
 import numpy as np
 import pytest
-from helpers import Oracle, make_params, SynthDB, build_fmi, have_ref, make_quirk_db
+import golden_workloads as gw
+from golden_workloads import golden_db
+from helpers import Oracle, make_params, make_quirk_db
 
 pytestmark = pytest.mark.gpu
 
@@ -12,19 +15,6 @@ pytestmark = pytest.mark.gpu
 def kb(built):
     import kaiju_b200
     return kaiju_b200
-
-
-def kfold_fasta(src, dst, k):
-    recs = []; cur = None
-    for l in open(src).read().split("\n"):
-        if l.startswith(">"):
-            cur = [l, []]; recs.append(cur)
-        elif cur is not None and l:
-            cur[1].append(l)
-    with open(dst, "w") as g:
-        for h, s in recs:
-            for _ in range(k):
-                g.write(h + "\n" + "\n".join(s) + "\n")
 
 
 @pytest.mark.parametrize("force_wide", [False, True])
@@ -49,8 +39,6 @@ def test_device_build_equals_host_transcoder(kb, golden, monkeypatch, force_wide
 
 def test_device_build_quirk_index(kb, tmp_path):
     """bwtlen = m * 2^16: the reference's checkpoint quirk constants and the k-mer table come out of the device build as on the host"""
-    if not have_ref():
-        pytest.skip("oracle/_ref (index builder) not available")
     fmi, nodes, reads = make_quirk_db(str(tmp_path))
     want = kb.host_index_checksums(fmi, nodes)
     clf = kb.Classifier(fmi, nodes, device=0, params=kb.make_params("mem"))
@@ -58,38 +46,28 @@ def test_device_build_quirk_index(kb, tmp_path):
     clf.close()
 
 
-@pytest.mark.parametrize("copies", [2, 3, 7])
-def test_scaled_index_equals_reference_built_kfold_index(kb, tmp_path, copies):
-    """kj_create_scaled(copies = K) == the index kaiju-mkbwt / kaiju-mkfmi build for the FASTA that holds every protein K times: same arrays in
-    HBM, same classification (MEM and Greedy); and MEM results equal those on the base index."""
-    if not have_ref():
-        pytest.skip("oracle/_ref (index builder) not available")
-    d = str(tmp_path)
-    db = SynthDB(3000, 11 + copies); db.write(d + "/base.faa", d + "/nodes.dmp")
-    kfold_fasta(d + "/base.faa", d + "/rep.faa", copies)
-    base = build_fmi(d + "/base.faa", d + "/base", threads=4); rep = build_fmi(d + "/rep.faa", d + "/rep", threads=4)
-    nodes = d + "/nodes.dmp"
-    want = kb.host_index_checksums(rep, nodes)
-    big = kb.Classifier(base, nodes, device=0, params=kb.make_params("mem"), copies=copies)
-    got = big.debug_index_checksums()
+@pytest.mark.parametrize("copies", list(gw.KFOLD_COPIES))
+def test_scaled_index_equals_reference_built_kfold_index(kb, golden, copies):
+    """kj_create_scaled(copies = K) == the index kaiju-mkbwt / kaiju-mkfmi build for the FASTA that holds every protein of the golden DB
+    K times: same arrays in HBM (the host transcoder's checksums of the reference-built index are stored), the reference's classification
+    on that index (MEM and Greedy, stored as a digest); and MEM results equal those on the base index."""
+    ans = gw.ref_answers()
+    big = kb.Classifier(golden.fmi, golden.nodes, device=0, params=kb.make_params("mem"), copies=copies)
+    got = big.debug_index_checksums(); want = ans["kfold%d_checksums" % copies]
     # the sampled-SA arrays differ in length by the reference's dropped last entry only: compare everything else exactly, the SA through results
     assert np.array_equal(got[[0, 1, 3, 4, 5, 6]], want[[0, 1, 3, 4, 5, 6]]), (got, want)
-    ref_built = kb.Classifier(rep, nodes, device=0, params=kb.make_params("mem"))
-    small = kb.Classifier(base, nodes, device=0, params=kb.make_params("mem"))
-    s1, o1, s2, o2 = db.reads(5, 0, 20000, 150, True)
-    orc = Oracle(rep, nodes)
+    small = kb.Classifier(golden.fmi, golden.nodes, device=0, params=kb.make_params("mem"))
+    s1, o1, s2, o2 = gw.kfold_reads()
     for mode in ("mem", "greedy"):
-        for c in (big, ref_built, small):
+        for c in (big, small):
             c.set_params(kb.make_params(mode))
-        a = big.classify(s1, o1, s2, o2); b = ref_built.classify(s1, o1, s2, o2)
-        assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]), mode
-        otax, obest = orc.classify_batch(make_params(mode), s1, o1, s2, o2)
-        assert np.array_equal(a[0], otax) and np.array_equal(a[1], obest), mode
+        a = big.classify(s1, o1, s2, o2)
+        assert gw.result_digest(*a) == str(ans["kfold%d_%s_sha256" % (copies, mode)]), mode
         if mode == "mem":
             c0 = small.classify(s1, o1, s2, o2)
             assert np.array_equal(a[0], c0[0]) and np.array_equal(a[1], c0[1])
     assert (a[0] != 0).mean() > 0.4
-    for c in (big, ref_built, small):
+    for c in (big, small):
         c.close()
 
 
@@ -120,18 +98,13 @@ def test_dense_taxon_indices(kb, golden):
     clf.close()
 
 
-def test_index_beyond_2_pow_32_rows(kb, tmp_path):
-    """A genuinely wide index (>= 2^32 BWT rows, not KJ_FORCE_WIDE): 23-fold scaling of a 2e8-row... too large for a unit test's
-    index builder, so a 7 M-row reference-built index is scaled 620 times (4.3e9 rows, ~20 GB in HBM); MEM results must equal the
-    base index's, which are checked against the oracle."""
-    if not have_ref():
-        pytest.skip("oracle/_ref (index builder) not available")
+def test_index_beyond_2_pow_32_rows(kb, golden):
+    """A genuinely wide index (>= 2^32 BWT rows, not KJ_FORCE_WIDE): the committed golden index scaled past 2^32 rows (~20 GB in HBM);
+    MEM results must equal the base index's, which are checked against the oracle."""
     import torch
     if torch.cuda.mem_get_info()[0] < (40 << 30):
         pytest.skip("needs 40 GB of free HBM")
-    d = str(tmp_path)
-    db = SynthDB(24000, 77); db.write(d + "/db.faa", d + "/nodes.dmp")
-    fmi = build_fmi(d + "/db.faa", d + "/db", threads=min(16, os.cpu_count())); nodes = d + "/nodes.dmp"
+    db = golden_db(); fmi, nodes = golden.fmi, golden.nodes
     small = kb.Classifier(fmi, nodes, device=0, params=kb.make_params("mem"))
     copies = (1 << 32) // small.bwtlen + 2
     big = kb.Classifier(fmi, nodes, device=0, params=kb.make_params("mem"), copies=copies)

@@ -1,11 +1,12 @@
 """GPU parity: the CUDA path called through the C ABI (libkaijub200.so) vs the committed reference outputs, the oracle on
 fresh seeded workloads, edge cases, and size-independent properties at large batch sizes.  Bit-exact (integer work)."""
 import ctypes as C
-import os, tempfile
+import os
 import numpy as np
 import pytest
 from conftest import GOLDEN_CONFIGS
-from helpers import Oracle, make_params, SynthDB, build_fmi, have_ref
+import golden_workloads as gw
+from helpers import Oracle, make_params, SynthDB
 
 pytestmark = pytest.mark.gpu
 
@@ -41,13 +42,9 @@ def test_gpu_matches_reference_golden(kb, gclf, golden, cfg, tag):
 
 
 @pytest.fixture(scope="module")
-def fresh(kb):
-    if not have_ref():
-        pytest.skip("oracle/_ref (index builder) not available")
-    d = tempfile.mkdtemp(prefix="kjgpu_")
-    db = SynthDB(20000, 5); db.write(d + "/db.faa", d + "/nodes.dmp")
-    fmi = build_fmi(d + "/db.faa", d + "/db", threads=min(16, os.cpu_count()))
-    return db, fmi, d + "/nodes.dmp"
+def fresh(kb, golden):
+    """Fresh seeded reads (tools/kjgen.c) from the DB of the committed golden index."""
+    return gw.golden_db(), golden.fmi, golden.nodes
 
 
 @pytest.mark.parametrize("kw", [dict(mode="mem"), dict(mode="mem", seg=False), dict(mode="mem", m=14), dict(mode="greedy"),
@@ -348,31 +345,11 @@ def test_file_ingest_on_device(kb, golden, tmp_path, monkeypatch, chunk):
 @pytest.mark.parametrize("chunk", ["1024", "20000", ""])
 def test_fastq_with_blank_lines(kb, golden, tmp_path, monkeypatch, chunk):
     """Empty lines between FASTQ records (and at the end of the file) are skipped where the reference's reader skips them (kaiju.cpp:288-289,
-    341-348); empty lines inside a record count as the record's lines.  Output == the output for the clean files == the reference binary's."""
-    import random
-    from helpers import run_ref_kaiju
+    341-348); empty lines inside a record count as the record's lines.  Output == the output for the clean files == the reference binary's
+    (stored in tests/golden/ref_answers.npz.xz)."""
     if chunk:
         monkeypatch.setenv("KJ_INGEST_CHUNK", chunk)
-    rnd = random.Random(11); db = SynthDB(800, 3)
-    s1, o1, s2, o2 = db.reads(93, 0, 500, 150, True)
-    r1 = [s1[int(o1[i]):int(o1[i + 1])].tobytes().decode() for i in range(500)]; r2 = [s2[int(o2[i]):int(o2[i + 1])].tobytes().decode() for i in range(500)]
-    def write(path, reads, blanks, mate):
-        with open(path, "w") as f:
-            if blanks:
-                f.write("\n\n")                                              # the file type comes from the first non-empty line
-            for i, sq in enumerate(reads):
-                if blanks and i and rnd.random() < 0.2:
-                    f.write("\n" * rnd.choice([1, 1, 2, 5]))
-                if blanks and i % 97 == 5:
-                    sq = ""                                                   # an empty sequence line is a line of the record, not a skipped one
-                    f.write("@r%d/%d\n\n+\n\n" % (i, mate))
-                    continue
-                f.write("@r%d/%d\n%s\n+\n%s\n" % (i, mate, sq, "I" * len(sq)))
-            if blanks:
-                f.write("\n\n\n")
-    clean1, clean2, b1, b2 = (str(tmp_path / x) for x in ("c1.fq", "c2.fq", "b1.fq", "b2.fq"))
-    r1c = [("" if i % 97 == 5 else x) for i, x in enumerate(r1)]; r2c = [("" if i % 97 == 5 else x) for i, x in enumerate(r2)]
-    write(clean1, r1c, False, 1); write(clean2, r2c, False, 2); write(b1, r1, True, 1); write(b2, r2, True, 2)
+    clean1, clean2, b1, b2 = gw.write_gpu_blank_line_fastq(str(tmp_path))
     clf = kb.Classifier(golden.fmi, golden.nodes, device=0, params=kb.make_params("greedy", e=3))
     outs = []
     for a, b in ((clean1, clean2), (b1, b2), (b1, clean2), (clean1, None), (b1, None)):
@@ -381,10 +358,10 @@ def test_fastq_with_blank_lines(kb, golden, tmp_path, monkeypatch, chunk):
         outs.append(open(o).read())
     assert outs[0] == outs[1] == outs[2] and outs[3] == outs[4] and outs[0].count("C\t") > 200
     clf.close()
-    if have_ref():
-        from helpers import parse_kaiju_output
-        assert parse_kaiju_output(outs[1]) == run_ref_kaiju(golden.nodes, golden.fmi, b1, b2, mode="greedy", e=3, threads=1)
-        assert parse_kaiju_output(outs[4]) == run_ref_kaiju(golden.nodes, golden.fmi, b1, None, mode="greedy", e=3, threads=1)
+    from helpers import parse_kaiju_output
+    ans = gw.ref_answers()                                                   # the reference binary's output for b1 (+ b2), stored
+    assert parse_kaiju_output(outs[1]) == gw.stored_run(ans, "gpu_blank_pe")
+    assert parse_kaiju_output(outs[4]) == gw.stored_run(ans, "gpu_blank_se")
 
 
 def test_per_taxon_counts(kb, golden, tmp_path, monkeypatch):
@@ -459,8 +436,6 @@ def test_index_with_bwtlen_multiple_of_65536(kb, tmp_path):
     """The reference's FM-index checkpoint quirk for bwtlen = m * 2^16 is reproduced on the GPU (oracle pinned to the reference for this
     case in tests/test_oracle_vs_ref.py), for the 32-bit, 64-bit and table-free kernels and through the device-native index file."""
     from helpers import make_quirk_db, pack_reads
-    if not have_ref():
-        pytest.skip("oracle/_ref (index builder) not available")
     fmi, nodes, reads = make_quirk_db(str(tmp_path))
     seq, off = pack_reads(reads); orc = Oracle(fmi, nodes)
     native = str(tmp_path / "q.kjb"); kb.write_native_index(fmi, nodes, native)
@@ -474,32 +449,15 @@ def test_index_with_bwtlen_multiple_of_65536(kb, tmp_path):
 
 
 def test_counts_table_equals_reference_kaiju2table(kb, golden, tmp_path):
-    """reads -> per-taxon counts in HBM -> kaiju2table report (kj_counts_table) == the reference's kaiju2table run on the per-read output file."""
-    import subprocess
-    from helpers import REF_DIR
-    k2t = os.path.join(REF_DIR, "kaiju2table")
-    if not os.path.exists(k2t):
-        pytest.skip("oracle/_ref/kaiju2table not built")
+    """reads -> per-taxon counts in HBM -> kaiju2table report (kj_counts_table) == the reference's kaiju2table run on the per-read output file
+    (the reference's reports are stored in tests/golden/kaiju2table_reports.json.gz)."""
     gold = os.path.dirname(golden.fmi); d = str(tmp_path)
-    # the golden taxonomy has no ranks: give every node a rank by depth and a name
-    par = {}
-    for l in open(golden.nodes):
-        p = l.split("\t|\t"); par[int(p[0])] = int(p[1])
-    ranks = ["no rank", "superkingdom", "phylum", "class", "order", "family", "genus", "species"]
-    def depth(x):
-        k = 0
-        while par[x] != x:
-            x = par[x]; k += 1
-        return k
-    with open(d + "/nodes.dmp", "w") as f, open(d + "/names.dmp", "w") as g:
-        for x in par:
-            f.write("%d\t|\t%d\t|\t%s\t|\n" % (x, par[x], ranks[min(depth(x), 7)])); g.write("%d\t|\ttaxon %d\t|\t\t|\tscientific name\t|\n" % (x, x))
+    gw.ranked_golden_taxonomy(golden.nodes, d)
+    reports = gw.k2t_reports()
     clf = kb.Classifier(golden.fmi, golden.nodes, device=0, params=kb.make_params("mem"))
     out = d + "/reads.tsv"
     clf.classify_files(os.path.join(gold, "pe150_1.fq.gz"), os.path.join(gold, "pe150_2.fq.gz"), out)
-    for o, flags in ((dict(rank="species"), ["-r", "species"]), (dict(rank="genus", filter_unclassified=True, full_path=True), ["-r", "genus", "-u", "-p"]),
-                     (dict(rank="phylum", min_read_count=5), ["-r", "phylum", "-c", "5"])):
-        subprocess.run([k2t, "-t", d + "/nodes.dmp", "-n", d + "/names.dmp", "-o", d + "/ref.tsv"] + flags + [out], check=True, stderr=subprocess.DEVNULL)
+    for i, (o, flags) in enumerate(gw.COUNTS_TABLE_OPTS):
         clf.counts_table(d + "/nodes.dmp", d + "/names.dmp", out, d + "/ours.tsv", **o)
-        assert open(d + "/ours.tsv").read() == open(d + "/ref.tsv").read(), o
+        assert open(d + "/ours.tsv").read() == reports["counts%d" % i].replace("{LABEL}", out), o
     clf.close()

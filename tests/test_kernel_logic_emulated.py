@@ -124,9 +124,7 @@ def test_native_index_file_roundtrip(emu, golden, tmp_path, monkeypatch):
 def test_emulated_kernel_on_index_with_bwtlen_multiple_of_65536(emu, built, tmp_path, monkeypatch):
     """The reference's checkpoint quirk (tests/test_oracle_vs_ref.py::test_bwtlen_multiple_of_65536) is reproduced by the device code:
     rank correction for the last 129 rows, in the k-mer table, in the SA walk, and the general 'recorded match' rule of maxMatches."""
-    from helpers import have_ref, make_quirk_db, pack_reads
-    if not have_ref():
-        pytest.skip("oracle/_ref (index builder) not available")
+    from helpers import make_quirk_db, pack_reads
     fmi, nodes, reads = make_quirk_db(str(tmp_path))
     seq, off = pack_reads(reads); orc = Oracle(fmi, nodes)
     for env in ({}, {"KJ_FORCE_WIDE": "1"}, {"KJ_KMER_K": "0"}):

@@ -1,75 +1,25 @@
-"""kj_table_write (kaiju2table's report from per-taxon counts) against the UNMODIFIED reference kaiju2table in oracle/_ref, byte for byte.
-CPU only; skipped when oracle/_ref/kaiju2table has not been built."""
-import os, random, subprocess
+"""kj_table_write (kaiju2table's report from per-taxon counts) against the UNMODIFIED reference kaiju2table, byte for byte: its reports
+for these inputs are stored in tests/golden/kaiju2table_reports.json.gz (tests/golden/make_golden_ref.py).  CPU only."""
+import random
 import numpy as np
 import pytest
-from helpers import REF_DIR
-
-K2T = os.path.join(REF_DIR, "kaiju2table")
-pytestmark = pytest.mark.skipif(not os.path.exists(K2T), reason="oracle/_ref/kaiju2table not built")
+import golden_workloads as gw
+from golden_workloads import make_taxonomy
 
 
-def make_taxonomy(d, rnd):
-    """root 1 -> superkingdoms 2 (Bacteria), 10239 (Viruses) -> phylum -> class -> order -> family -> genus -> species, plus 'no rank' nodes."""
-    ranks = ["superkingdom", "phylum", "class", "order", "family", "genus", "species"]
-    nodes = {1: (1, "no rank")}; names = {1: "root"}; nxt = [20000]; leaves = []
-    def grow(parent, depth, tag):
-        if depth == len(ranks):
-            leaves.append(parent); return
-        for k in range(rnd.choice([1, 2, 2, 3])):
-            nid = nxt[0]; nxt[0] += rnd.choice([1, 3, 7]); nodes[nid] = (parent, ranks[depth]); names[nid] = "%s %s%d" % (tag, ranks[depth][:3], nid)
-            if depth == 3 and k == 0:                      # an unranked node in the lineage
-                mid = nxt[0]; nxt[0] += 1; nodes[mid] = (nid, "no rank"); names[mid] = "%s clade%d" % (tag, mid); grow(mid, depth + 1, tag)
-            else:
-                grow(nid, depth + 1, tag)
-    nodes[2] = (1, "superkingdom"); names[2] = "Bacteria"; nodes[10239] = (1, "superkingdom"); names[10239] = "Viruses"
-    grow(2, 1, "Bac"); grow(10239, 1, "Vir")
-    with open(d + "/nodes.dmp", "w") as f:
-        for nid, (par, rk) in nodes.items():
-            f.write("%d\t|\t%d\t|\t%s\t|\t\t|\n" % (nid, par, rk))
-    with open(d + "/names.dmp", "w") as f:
-        for nid, nm in names.items():
-            if nid % 11 == 5:
-                continue                                   # some taxa have no name -> "taxonid:<id>"
-            f.write("%d\t|\t%s synonym\t|\t\t|\tsynonym\t|\n" % (nid, nm))
-            f.write("%d\t|\t%s\t|\t\t|\tscientific name\t|\n" % (nid, nm))
-    return nodes, leaves
-
-
-OPTS = [dict(rank="species"), dict(rank="genus", expand_viruses=True), dict(rank="family", filter_unclassified=True), dict(rank="phylum", min_percent=2.5),
-        dict(rank="species", min_read_count=40), dict(rank="genus", full_path=True), dict(rank="species", rank_list="superkingdom,phylum,genus,species", expand_viruses=True),
-        dict(rank="class", filter_unclassified=True, min_percent=0.5, expand_viruses=True)]
-
-
-@pytest.mark.parametrize("o", OPTS)
+@pytest.mark.parametrize("o", gw.TABLE_OPTS)
 def test_table_equals_reference_kaiju2table(built, tmp_path, o):
     import kaiju_b200 as kb
-    rnd = random.Random(11); d = str(tmp_path)
-    nodes, leaves = make_taxonomy(d, rnd)
-    # a kaiju output file: classified reads on leaves, inner nodes and a taxon that is missing from nodes.dmp; unclassified reads
-    pool = leaves + rnd.sample(sorted(nodes), 12) + [999999]
-    weights = [rnd.choice([1, 1, 2, 5, 20, 80]) for _ in pool]
-    reads = rnd.choices(pool, weights, k=6000) + [0] * 1500
-    rnd.shuffle(reads)
-    with open(d + "/in.tsv", "w") as f:
-        for i, t in enumerate(reads):
-            f.write("C\tr%d\t%d\n" % (i, t) if t else "U\tr%d\t0\n" % i)
-    flags = ["-r", o["rank"]]
-    flags += ["-e"] if o.get("expand_viruses") else []
-    flags += ["-u"] if o.get("filter_unclassified") else []
-    flags += ["-p"] if o.get("full_path") else []
-    flags += ["-m", str(o["min_percent"])] if "min_percent" in o else []
-    flags += ["-c", str(o["min_read_count"])] if "min_read_count" in o else []
-    flags += ["-l", o["rank_list"]] if "rank_list" in o else []
-    subprocess.run([K2T, "-t", d + "/nodes.dmp", "-n", d + "/names.dmp", "-o", d + "/ref.tsv"] + flags + [d + "/in.tsv"], check=True, stderr=subprocess.DEVNULL)
+    d = str(tmp_path); i = gw.TABLE_OPTS.index(o); reports = gw.k2t_reports()
+    reads, rnd = gw.table_input(d, o)
+    label = d + "/in.tsv"
     ids, cnt = np.unique(np.array(reads, dtype=np.uint64), return_counts=True)
     perm = rnd.sample(range(len(ids)), len(ids))          # the order of the count vector must not matter
-    kb.write_table(ids[perm], cnt[perm], d + "/nodes.dmp", d + "/names.dmp", d + "/in.tsv", d + "/ours.tsv", **o)
-    assert open(d + "/ours.tsv").read() == open(d + "/ref.tsv").read()
+    kb.write_table(ids[perm], cnt[perm], d + "/nodes.dmp", d + "/names.dmp", label, d + "/ours.tsv", **o)
+    assert open(d + "/ours.tsv").read() == reports["table%d" % i].replace("{LABEL}", label)
     # two data sets in one report (kaiju2table in1 in2): second call appends
-    subprocess.run([K2T, "-t", d + "/nodes.dmp", "-n", d + "/names.dmp", "-o", d + "/ref2.tsv"] + flags + [d + "/in.tsv", d + "/in.tsv"], check=True, stderr=subprocess.DEVNULL)
-    kb.write_table(ids, cnt, d + "/nodes.dmp", d + "/names.dmp", d + "/in.tsv", d + "/ours.tsv", append=True, **o)
-    assert open(d + "/ours.tsv").read() == open(d + "/ref2.tsv").read()
+    kb.write_table(ids, cnt, d + "/nodes.dmp", d + "/names.dmp", label, d + "/ours.tsv", append=True, **o)
+    assert open(d + "/ours.tsv").read() == reports["table%d_twice" % i].replace("{LABEL}", label)
 
 
 def test_table_argument_errors(built, tmp_path):
