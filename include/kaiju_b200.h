@@ -209,6 +209,31 @@ int kj_counts_table(kj_ctx *ctx, const char *nodes_dmp, const char *names_dmp, c
  * library enlarges the ring, so repeating the call succeeds -- kj_classify() does that internally. */
 int kj_check_errors(kj_ctx *ctx);
 
+/* --- index construction: protein FASTA -> .fmi (what `kaiju-mkbwt -a ALPHABET -e E` followed by `kaiju-mkfmi` writes, byte for byte) --- */
+/* The generalized suffix array (every sequence followed by its own terminator; terminators sort below all letters and among
+ * themselves by input order), the BWT, the sampled suffix array and the compact FM index are all built on the device: prefix
+ * doubling with hand-written radix sorts, re-sorting only the suffixes that are still tied.  The host parses the FASTA with
+ * kaiju-mkbwt's rules (readFasta.c, sequence.c) and writes the files.  Limits: fewer than 2^32 rows (residues + sequences),
+ * at most 24 letters.  A '*' (the terminator character) inside a sequence is refused: kaiju-mkbwt reads it as a sequence end
+ * and writes a BWT shorter than its own header.  Bytes >= 0x80 are skipped like other non-letters. */
+#define KJ_MKFMI_MAX_ROUNDS 40
+typedef struct {
+    int32_t chpt_exp;             /* -e: a suffix-array sample every 2^chpt_exp rows (0..16; kaiju-makedb uses 5, tests 3)      */
+    const char *alphabet;         /* -a: the letters (NULL = "ACDEFGHIKLMNPQRSTVWY"), or "protein" (= the 20 residues + X)     */
+    int32_t write_bwt_sa;         /* also write <prefix>.bwt and <prefix>.sa as kaiju-mkbwt does                              */
+} kj_mkfmi_opts;
+typedef struct {
+    int64_t bwtlen;               /* rows: residues + sequences                                                                */
+    int32_t nseq;
+    int32_t sort_rounds;          /* radix-sorted rounds: the initial one on packed letters + the prefix-doubling ones        */
+    uint64_t round_items[KJ_MKFMI_MAX_ROUNDS];   /* suffixes sorted in each round (round 0 = all of them)                   */
+    uint64_t sort_bytes;          /* bytes the sort kernels read and write (keys, values, histograms), over all rounds        */
+    double parse_ms, upload_ms, sort_ms, assemble_ms, write_ms;   /* wall time of the stages                                  */
+} kj_mkfmi_stats;
+/* KJ_ERR_UNSUPPORTED: >= 2^32 rows, more than 24 letters, no sequence in the input, '*' in a sequence; KJ_ERR_NOMEM: the device
+ * memory estimate (about 45 bytes per row) exceeds the free memory; KJ_ERR_NO_DEVICE without a GPU.  stats may be NULL. */
+int kj_mkfmi(const char *faa_path, const char *out_prefix, const kj_mkfmi_opts *opts, int device, kj_mkfmi_stats *stats);
+
 /* --- introspection --- */
 const char *kj_last_error(void);                  /* thread-local text of the last failure          */
 uint64_t kj_kernel_launches(const kj_ctx *ctx);   /* number of kernels this context has launched    */

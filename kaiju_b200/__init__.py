@@ -39,6 +39,16 @@ class KjTableOpts(C.Structure):
                 ("filter_unclassified", C.c_int32), ("full_path", C.c_int32), ("rank_list", C.c_char_p)]
 
 
+class KjMkfmiOpts(C.Structure):
+    _fields_ = [("chpt_exp", C.c_int32), ("alphabet", C.c_char_p), ("write_bwt_sa", C.c_int32)]
+
+
+class KjMkfmiStats(C.Structure):
+    _fields_ = [("bwtlen", C.c_int64), ("nseq", C.c_int32), ("sort_rounds", C.c_int32), ("round_items", C.c_uint64 * 40),
+                ("sort_bytes", C.c_uint64), ("parse_ms", C.c_double), ("upload_ms", C.c_double), ("sort_ms", C.c_double),
+                ("assemble_ms", C.c_double), ("write_ms", C.c_double)]
+
+
 class KaijuError(RuntimeError):
     pass
 
@@ -94,6 +104,8 @@ def lib():
         L.kj_check_errors.argtypes = [C.c_void_p]
         L.kj_launch_geometry.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
         L.kj_version.restype = C.c_int
+        if hasattr(L, "kj_mkfmi"):
+            L.kj_mkfmi.argtypes = [C.c_char_p, C.c_char_p, C.POINTER(KjMkfmiOpts), C.c_int, C.POINTER(KjMkfmiStats)]
         _lib = L
     return _lib
 
@@ -154,6 +166,16 @@ def write_native_index(fmi_path, nodes_path, out_path):
             L.kj_nodes_free(nodes)
     finally:
         L.kj_fmi_free(fmi)
+
+
+def build_index(faa, prefix, exponent=3, alphabet="ACDEFGHIKLMNPQRSTVWY", device=0, write_bwt_sa=False):
+    """Protein FASTA -> <prefix>.fmi on the GPU, byte for byte what `kaiju-mkbwt -a ALPHABET -e EXPONENT` + `kaiju-mkfmi` write
+    (kj_mkfmi; alphabet may also be "protein").  With write_bwt_sa also <prefix>.bwt and <prefix>.sa.  Returns the build statistics."""
+    o = KjMkfmiOpts(int(exponent), alphabet.encode() if alphabet else None, 1 if write_bwt_sa else 0); st = KjMkfmiStats()
+    _check(lib().kj_mkfmi(os.fspath(faa).encode(), os.fspath(prefix).encode(), C.byref(o), int(device), C.byref(st)))
+    return {"bwtlen": int(st.bwtlen), "nseq": int(st.nseq), "sort_rounds": int(st.sort_rounds),
+            "round_items": [int(st.round_items[i]) for i in range(st.sort_rounds)], "sort_bytes": int(st.sort_bytes),
+            "parse_ms": st.parse_ms, "upload_ms": st.upload_ms, "sort_ms": st.sort_ms, "assemble_ms": st.assemble_ms, "write_ms": st.write_ms}
 
 
 def device_count():

@@ -1,5 +1,6 @@
 // kj_cli.cpp -- `kaiju-b200`: the reference's command-line surface (src/kaiju.cpp:74-202, usage 430-451) on top of the C ABI.
 //   kaiju-b200 -t nodes.dmp -f db.fmi -i reads.fastq [-j reads2.fastq] [-a mem|greedy] [-m -s -e -E -l] [-x|-X] [-o out] [-z N] [-v]
+//   kaiju-b200 -M mkfmi -i db.faa -o prefix [-e 3] [-a ALPHABET] [-d N]      (index construction on the GPU)
 // Output: "C\t<name>\t<taxid>\n" / "U\t<name>\t0\n" (ConsumerThread.cpp:724-739), in INPUT order.
 // Host glue only: option parsing; kj_classify_files() reads FASTA/FASTQ(.gz), parses it on the device with the reference's name
 // trimming (kaiju.cpp:318-335) and strip() (util.cpp:26-33), classifies and formats the output.  -z is accepted and ignored (the GPU replaces the consumer threads); -p = protein input; with -v
@@ -158,6 +159,30 @@ int run_verbose(kj_ctx* ctx, kj_fmi* fmi, const kj_params& P, const std::string&
 }  // namespace
 
 static void die(const std::string& m) { fprintf(stderr, "Error: %s\n\n", m.c_str()); exit(EXIT_FAILURE); }
+// -M mkfmi: protein FASTA -> <prefix>.fmi on the GPU (kj_mkfmi), what `kaiju-mkbwt -a ALPHABET -e E -o prefix db.faa` + `kaiju-mkfmi prefix`
+// write; with -w (and -t) the new index is also transcoded into a device-native index file.  Exit status 1 on any error.
+static int run_mkfmi(const std::string& in, const std::string& prefix, const char* a_arg, const char* e_arg, const std::string& dev,
+                     const std::string& nodes_fn, const std::string& native_out) {
+    if (in.empty() || prefix.empty()) die("-M mkfmi needs the protein FASTA (-i) and the output prefix (-o)");
+    if (!native_out.empty() && nodes_fn.empty()) die("-w after -M mkfmi needs nodes.dmp (-t)");
+    kj_mkfmi_opts o; memset(&o, 0, sizeof o);
+    o.chpt_exp = 3; o.alphabet = a_arg;
+    if (e_arg) { char* end = nullptr; const long v = strtol(e_arg, &end, 10); if (!*e_arg || *end || v < 0 || v > 16) die("-e (suffix array sampling exponent) must be 0..16"); o.chpt_exp = (int32_t)v; }
+    char* end = nullptr; const long d = strtol(dev.c_str(), &end, 10);
+    if (dev.empty() || *end || d < 0) die("-M mkfmi takes one device number (-d N)");
+    kj_mkfmi_stats st;
+    if (kj_mkfmi(in.c_str(), prefix.c_str(), &o, (int)d, &st) != KJ_OK) die(kj_last_error());
+    fprintf(stderr, "%s.fmi: %lld rows, %d sequences, %d sort rounds; %.1f ms parse, %.1f ms upload, %.1f ms sort, %.1f ms assembly, %.1f ms write\n",
+            prefix.c_str(), (long long)st.bwtlen, st.nseq, st.sort_rounds, st.parse_ms, st.upload_ms, st.sort_ms, st.assemble_ms, st.write_ms);
+    if (!native_out.empty()) {
+        kj_fmi* fmi = nullptr; kj_nodes* nodes = nullptr;
+        if (kj_nodes_load(nodes_fn.c_str(), &nodes) != KJ_OK || kj_fmi_load((prefix + ".fmi").c_str(), &fmi) != KJ_OK) die(kj_last_error());
+        kj_index_view iv; kj_taxonomy_view tv; kj_fmi_view(fmi, &iv); kj_nodes_view(nodes, &tv);
+        if (kj_native_index_write(&iv, &tv, native_out.c_str()) != KJ_OK) die(kj_last_error());
+        kj_fmi_free(fmi); kj_nodes_free(nodes);
+    }
+    return EXIT_SUCCESS;
+}
 static void usage(const char* prog) {
     fprintf(stderr, "kaiju-b200 (B200-native classification path of Kaiju)\n\nUsage:\n   %s -t nodes.dmp -f kaiju_db.fmi -i reads.fastq [-j reads2.fastq]\n\n"
                     "Mandatory arguments:\n   -t FILENAME   Name of nodes.dmp file\n   -f FILENAME   Name of database (.fmi) file\n   -i FILENAME   Name of input file containing reads in FASTA or FASTQ format\n\n"
@@ -165,16 +190,17 @@ static void usage(const char* prog) {
                     "   -z INT        accepted for compatibility (ignored: the GPU replaces the worker threads)\n   -a STRING     Run mode, either \"mem\"  or \"greedy\" (default: greedy)\n"
                     "   -e INT        Number of mismatches allowed in Greedy mode (default: 3)\n   -m INT        Minimum match length (default: 11)\n   -s INT        Minimum match score in Greedy mode (default: 65)\n"
                     "   -E FLOAT      Minimum E-value in Greedy mode (default: 0.01)\n   -x            Enable SEG low complexity filter (enabled by default)\n   -X            Disable SEG low complexity filter\n"
-                    "   -w FILENAME   Write the device-native index file for -t/-f and exit; such a file can then be given as -f (no -t needed, no transcode at start-up)\n   -T FILENAME   Also write kaiju2table's summary (reads per taxon of rank -r, default species; needs -N names.dmp) from the counts kept on the GPU\n   -p            Input sequences are protein sequences\n   -v            Enable verbose output (adds the match length/score, the matching taxon ids, accession numbers and fragment sequences)\n   -M STRING     front-end: \"kaijux\" (as kaiju, but reports the names of the matching database sequences; no -t) or \"kaijup\" (the same for protein reads)\n   -d LIST       CUDA device ordinal(s): one number, a comma-separated list, or \"all\" (default 0).  With several devices the data sets of the\n                 -i/-j/-o lists are classified in parallel, one context (index replica) per device\n", prog);
+                    "   -w FILENAME   Write the device-native index file for -t/-f and exit; such a file can then be given as -f (no -t needed, no transcode at start-up)\n   -T FILENAME   Also write kaiju2table's summary (reads per taxon of rank -r, default species; needs -N names.dmp) from the counts kept on the GPU\n   -p            Input sequences are protein sequences\n   -v            Enable verbose output (adds the match length/score, the matching taxon ids, accession numbers and fragment sequences)\n   -M STRING     front-end: \"kaijux\" (as kaiju, but reports the names of the matching database sequences; no -t) or \"kaijup\" (the same for protein reads),\n                 or \"mkfmi\": build the index <-o>.fmi from the protein FASTA -i on the GPU, as kaiju-mkbwt + kaiju-mkfmi do (no -f; -e = suffix\n                 array sampling exponent, default 3; -a = alphabet, default ACDEFGHIKLMNPQRSTVWY, or \"protein\"; -w FILE -t nodes.dmp also writes a native index)\n   -d LIST       CUDA device ordinal(s): one number, a comma-separated list, or \"all\" (default 0).  With several devices the data sets of the\n                 -i/-j/-o lists are classified in parallel, one context (index replica) per device\n", prog);
     exit(EXIT_FAILURE);
 }
 
 int main(int argc, char** argv) {
     kj_params P; P.mode = 1; P.min_fragment_length = 11; P.mismatches = 3; P.min_score = 65; P.seed_length = 7; P.use_evalue = 1; P.min_evalue = 0.01; P.seg = 1; P.input_is_protein = 0; P.name_mode = 0;
     std::string nodes_fn, fmi_fn, in1, in2, out_fn, native_out, table_fn, table_rank = "species", names_fn; bool verbose = false; std::string device_arg = "0", frontend; int c;
+    const char* a_arg = nullptr; const char* e_arg = nullptr;       // -a / -e: run mode and mismatches, or with -M mkfmi alphabet and SA exponent
     while ((c = getopt(argc, argv, "a:hd:pxXvn:m:e:E:l:t:f:i:j:s:z:o:w:T:r:N:M:")) != -1) {
         switch (c) {
-            case 'a': if (!strcmp(optarg, "mem")) { P.mode = 0; P.use_evalue = 0; } else if (!strcmp(optarg, "greedy")) P.mode = 1; else { fprintf(stderr, "-a must be a valid mode.\n"); usage(argv[0]); } break;
+            case 'a': a_arg = optarg; break;
             case 'h': usage(argv[0]); break;
             case 'd': device_arg = optarg; break;
             case 'v': verbose = true; break;
@@ -193,7 +219,7 @@ int main(int argc, char** argv) {
             case 'l': { int v = atoi(optarg); if (v < 7) { die("Seed length must be >= 7."); } P.seed_length = (uint32_t)v; break; }
             case 's': { int v = atoi(optarg); if (v <= 0) die("Min Score (-s) must be greater than 0."); P.min_score = (uint32_t)v; break; }
             case 'm': { int v = atoi(optarg); if (v <= 0) die("Min fragment length (-m) must be greater than 0."); P.min_fragment_length = (uint32_t)v; break; }
-            case 'e': { int v = atoi(optarg); if (v < 0) die("Number of mismatches must be >= 0."); P.mismatches = (uint32_t)v; break; }
+            case 'e': e_arg = optarg; break;
             case 'E': { P.min_evalue = atof(optarg); if (P.min_evalue <= 0.0) die("E-value threshold must be greater than 0."); break; }
             case 'z': { if (atoi(optarg) <= 0) die("Number of threads (-z) must be greater than 0."); break; }
             case 'n': break;
@@ -201,10 +227,13 @@ int main(int argc, char** argv) {
             default: usage(argv[0]);
         }
     }
+    if (frontend == "mkfmi") return run_mkfmi(in1, out_fn, a_arg, e_arg, device_arg, nodes_fn, native_out);
+    if (a_arg) { if (!strcmp(a_arg, "mem")) { P.mode = 0; P.use_evalue = 0; } else if (!strcmp(a_arg, "greedy")) P.mode = 1; else { fprintf(stderr, "-a must be a valid mode.\n"); usage(argv[0]); } }
+    if (e_arg) { int v = atoi(e_arg); if (v < 0) die("Number of mismatches must be >= 0."); P.mismatches = (uint32_t)v; }
     if (fmi_fn.empty()) { fprintf(stderr, "Error: Please specify the location of the FMI file, using the -f option.\n\n"); usage(argv[0]); }
     { const char* b = strrchr(argv[0], '/'); const std::string prog = b ? b + 1 : argv[0]; if (frontend.empty() && (prog == "kaijux" || prog == "kaijup")) frontend = prog; }
     if (!frontend.empty()) {      // -M kaijux | kaijup (or invoked under that name): report the names of the matching database sequences, no taxonomy
-        if (frontend != "kaijux" && frontend != "kaijup") die("-M must be kaijux or kaijup");
+        if (frontend != "kaijux" && frontend != "kaijup") die("-M must be kaijux, kaijup or mkfmi");
         if (in1.empty()) { fprintf(stderr, "Error: Please specify the location of the input file, using the -i option.\n\n"); usage(argv[0]); }
         if (frontend == "kaijup" && !in2.empty()) die("kaijup takes one input file");
         return run_name_frontend(frontend == "kaijup", P, fmi_fn, in1, in2, out_fn, atoi(device_arg.c_str()));
